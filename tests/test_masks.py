@@ -22,7 +22,7 @@ def _gold():
 
 def _unpack(packed, shape):
     n = int(np.prod(shape))
-    return torch.from_numpy(np.unpackbits(packed)[:n].reshape(shape).astype(np.int64))
+    return torch.from_numpy(np.unpackbits(np.asarray(packed))[:n].reshape(shape).astype(np.int64))
 
 
 def _parsing_input(h, w, seed):
@@ -42,7 +42,7 @@ def test_oracle_face_parsing_matches_reference(name):
     with torch.no_grad():
         masks, y, labels = R.face_parsing_forward(StubBiSeNet(), x)
     assert torch.allclose(F.interpolate(((x - torch.tensor(R.PARSING_MEAN)[None, :, None, None]) / torch.tensor(R.PARSING_STD)[None, :, None, None]),
-                                        size=(512, 512), mode="bilinear")[:, :, ::8, ::8], g["x512_s8"], atol=1e-6)
+                                        size=(512, 512), mode="bilinear")[:, :, ::16, ::16], g["x512_s16"], atol=1e-6)
     for m, packed, total in zip(masks, g["masks_packed"], g["masks_sum"]):
         ref = _unpack(packed, m.shape)
         assert int(ref.sum()) == total
@@ -60,7 +60,7 @@ def test_oracle_get_mask_matches_reference(name):
     with torch.no_grad():
         matte = R.modnet_get_mask(StubMODNet(), img)
     assert matte.shape == (1, 1, h, w)
-    assert torch.allclose(matte[:, :, ::2, ::2], g["matte_s2"], atol=1e-6)
+    assert torch.allclose(matte[:, :, ::4, ::4], g["matte_s4"], atol=1e-6)
 
 
 def test_face_parsing_rejects_mask_types_like_the_reference():
@@ -150,7 +150,7 @@ def test_get_mask_matches_reference_fixture(name):
     assert matte.shape == (1, 1, h, w)
     # the stand-in network runs in torch on the GPU (rounds differently from the CPU run of the fixture); the two area resizes
     # around it are checked exactly in test_resize_area_kernel
-    assert (matte.cpu()[:, :, ::2, ::2] - g["matte_s2"]).abs().max().item() <= 2e-4
+    assert (matte.cpu()[:, :, ::4, ::4] - g["matte_s4"]).abs().max().item() <= 2e-4
 
 
 @pytest.mark.gpu
